@@ -9,6 +9,7 @@ than the 126 MB L2, so nothing is cache-resident between steps).
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
          --master-port P bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference ...      # the reference's own CPU block on the host cores
+  python bench.py ... --dump-outputs DIR    # also write what the last timed step computed, DIR/<name>.npy
 
 The ONE JSON line carries the headline workload in the contract's top-level keys and, under
 "configs", one record per BASELINE.json config measured in the same run (each with its own
@@ -87,6 +88,10 @@ DTYPE_CODES = {"float32": 0, "complex_float32": 1, "float64": 2, "complex_float6
                "int16": 6, "complex_int16": 7, "int32": 8, "complex_int32": 9, "int64": 10, "complex_int64": 11}
 # CPU sample per host thread (log2 samples), sized so one pass takes ~1-2 s on the box's cores
 CPU_LOG2 = {"headline": 22, "c1": 22, "c1_real": 22, "c2": 22, "c3": 22, "c5": 20, "c3_i16": 22}
+# --dump-outputs keeps at most this many rows of each output (a workload returns at most two complex outputs: at most
+# 2 x (16 MiB of float64 values + 8 MiB of row numbers) = 48 MiB per run)
+DUMP_ROWS = 1 << 20
+DUMP_SEED = 0xD0D0
 
 
 def measured_peaks():
@@ -352,6 +357,28 @@ def timed_region(ctx: Ctx, step, steps: int, warmup: int, kernel_events: bool = 
     return elapsed / steps, kernel_ms, clocks
 
 
+def dump_outputs(path: str, outputs: dict) -> None:
+    """--dump-outputs: each CUDA tensor of `outputs` (what the timed path returned in its last step, [..., ncomp]) as
+    path/<name>.npy, rows x ncomp -- float32 for float32, int8 and int16 data (exact), float64 otherwise -- and the row
+    numbers it holds as path/<name>_rows.npy (float64).  An output longer than DUMP_ROWS keeps a fixed sample: one row at a
+    seeded place in each of DUMP_ROWS equal spans.  The inputs are seeded as well, so two builds run with the same
+    arguments can be compared row for row."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.reshape(-1, t.shape[-1])
+        n = t.shape[0]
+        rows = np.arange(n, dtype=np.int64)
+        if n > DUMP_ROWS:
+            lo = np.arange(DUMP_ROWS + 1, dtype=np.int64) * n // DUMP_ROWS
+            rows = lo[:-1] + (np.random.default_rng(DUMP_SEED).random(DUMP_ROWS) * np.diff(lo)).astype(np.int64)
+        vals = t.index_select(0, torch.from_numpy(rows).to(t.device)).cpu().numpy()
+        exact32 = vals.dtype == np.float32 or (vals.dtype.kind == "i" and vals.itemsize <= 2)
+        np.save(os.path.join(path, f"{name}.npy"), vals.astype(np.float32 if exact32 else np.float64))
+        np.save(os.path.join(path, f"{name}_rows.npy"), rows.astype(np.float64))
+
+
 def kernel_note(kernel: str) -> str:
     if kernel == "fir_os32x_kernel":
         return ("spectral resampler (one 1024-point forward + one 1536-point inverse transform per block): one pass over "
@@ -407,7 +434,7 @@ def halo_check(ctx: Ctx, fir, buf, out, K: int, M: int, L: int, code: int, taps,
 
 
 def bench_stream(ctx: Ctx, name: str, steps: int, warmup: int, e2e: bool, cpu: bool, log2n: int | None = None,
-                 split: str = "weak", ntaps: int | None = None, check: bool = True) -> dict:
+                 split: str = "weak", ntaps: int | None = None, check: bool = True, dump: str | None = None) -> dict:
     """One FIR stream workload.  split = "weak": 2^log2n samples per GPU; "strong": one 2^log2n-sample stream over
     all ranks.  Returns the record (value, roofline, cpu_baseline, e2e, ...)."""
     torch = ctx.torch
@@ -461,6 +488,8 @@ def bench_stream(ctx: Ctx, name: str, steps: int, warmup: int, e2e: bool, cpu: b
         assert c == n_seg and p == out_cap, (c, p, n_seg, out_cap)
 
     ms_per_step, kernel_ms, clocks = timed_region(ctx, step, steps, warmup)
+    if dump and rank == 0:
+        dump_outputs(dump, {"fir_out": out})
     value = world * n_seg / (ms_per_step * 1e-3) / 1e6
     halo = halo_check(ctx, fir, buf, out, K, M, L, code, taps, tt) if check else "skipped"
 
@@ -547,7 +576,8 @@ def bench_stream(ctx: Ctx, name: str, steps: int, warmup: int, e2e: bool, cpu: b
             "halo": {"mode": halo_mode, "check": halo}, "parity": parity}
 
 
-def bench_fft(ctx: Ctx, name: str, steps: int, warmup: int, e2e: bool, cpu: bool, log2n: int | None = None) -> dict:
+def bench_fft(ctx: Ctx, name: str, steps: int, warmup: int, e2e: bool, cpu: bool, log2n: int | None = None,
+              dump: str | None = None) -> dict:
     """BASELINE config 4: /comms/fft 4096-point forward then inverse over 2^28 samples (per GPU: transforms are
     independent, the batch is sharded with no exchange).  One step = two passes (2 launches); value counts samples per pass."""
     torch = ctx.torch
@@ -571,6 +601,8 @@ def bench_fft(ctx: Ctx, name: str, steps: int, warmup: int, e2e: bool, cpu: bool
         record(1)
 
     ms, kernel_ms, clocks = timed_region(ctx, step, steps, warmup)
+    if dump and ctx.rank == 0:
+        dump_outputs(dump, {"fft_forward": X, "fft_inverse": y})
     value = ctx.world * 2 * total / (ms * 1e-3) / 1e6
     esz = x.element_size() * 2
     achieved = 2 * esz * total * 2 / (kernel_ms * 1e-3) / 1e9    # (read + write) x two passes
@@ -634,7 +666,8 @@ def bench_fft(ctx: Ctx, name: str, steps: int, warmup: int, e2e: bool, cpu: bool
             "cpu_baseline": cpu_rec, "e2e": e2e_rec, "gpu_launches": 2 * steps, "clocks": clocks, "parity": parity}
 
 
-def bench_bank(ctx: Ctx, steps: int, warmup: int, e2e: bool, cpu: bool, channels: int | None = None, log2n: int | None = None) -> dict:
+def bench_bank(ctx: Ctx, steps: int, warmup: int, e2e: bool, cpu: bool, channels: int | None = None, log2n: int | None = None,
+               dump: str | None = None) -> dict:
     """BASELINE config 5: 1024-channel filter bank, one 1024-tap complex band-pass per channel, 2^20 samples per
     channel, channels sharded over the ranks (no exchange: SURVEY.md 8e).  Strong scaling: the bank is fixed, every
     rank takes 1024/N channels.  One step = one b200c_fir_bank_run over the rank's channels (one launch)."""
@@ -667,6 +700,8 @@ def bench_bank(ctx: Ctx, steps: int, warmup: int, e2e: bool, cpu: bool, channels
         assert (cons, prod) == (n_new, n_new), (cons, prod)
 
     ms, kernel_ms, clocks = timed_region(ctx, step, steps, warmup)
+    if dump and ctx.rank == 0:
+        dump_outputs(dump, {"bank_out": out})
     total = nchan_total * n_new
     value = total / (ms * 1e-3) / 1e6
     # parity: this rank's first channel against a single-stream filter and against the CPU oracle (sampled window)
@@ -776,7 +811,13 @@ def main():
     ap.add_argument("--log2-samples", type=int, default=None, help="override samples per GPU (debug)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "headline_blocks"):
+        ap.error("--dump-outputs is not available for --impl reference or --workload headline_blocks")
     if args.impl == "reference":
         return reference_arm(args)
     args.warmup = max(args.warmup, 3)
@@ -784,18 +825,20 @@ def main():
     e2e, cpu = not args.no_e2e, not args.no_cpu
 
     ctx = Ctx()
+    dump = args.dump_outputs
     if args.workload == "headline_blocks":
         main_rec = bench_blocks(ctx)
     elif args.workload in ("c4", "c4_i16"):
-        main_rec = bench_fft(ctx, args.workload, args.steps, args.warmup, e2e, cpu, args.log2_samples)
+        main_rec = bench_fft(ctx, args.workload, args.steps, args.warmup, e2e, cpu, args.log2_samples, dump=dump)
     elif args.workload == "c5_bank":
-        main_rec = bench_bank(ctx, args.steps, args.warmup, e2e, cpu and ctx.world == 1, args.channels, args.log2_samples)
+        main_rec = bench_bank(ctx, args.steps, args.warmup, e2e, cpu and ctx.world == 1, args.channels, args.log2_samples,
+                              dump=dump)
     else:
         main_rec = bench_stream(ctx, args.workload, args.steps, args.warmup, e2e, cpu and ctx.world == 1, args.log2_samples,
-                                ntaps=args.ntaps)
+                                ntaps=args.ntaps, dump=dump)
     configs = []
     if want_configs:
-        sub_steps, sub_warm = max(3, min(args.steps, 5)), 3
+        sub_steps, sub_warm = args.steps, 3
         if ctx.world == 1:
             plan = [("stream", "c1", 28, "weak"), ("stream", "c2", 28, "weak"), ("stream", "c3", 30, "strong"),
                     ("fft", "c4"), ("fft", "c4_i16"), ("bank",), ("blocks",)]

@@ -212,14 +212,19 @@ def test_multithreaded_driver_equals_single(oracle):
 
 
 def test_fir_golden_fixtures(oracle):
-    """tests/golden/fir_*.npz are outputs of the REFERENCE's compiled block (make_golden.py, `source` field)."""
+    """tests/golden/fir_*.npz are outputs of the REFERENCE's compiled block (make_golden.py, `source` field): one work()
+    call, and the first 500 inputs as a burst flushed by a frame-end label (the oracle's zero_tail=True)."""
     files = sorted(f for f in os.listdir(GOLDEN) if f.startswith("fir_") and f.endswith(".npz"))
     assert files
     for fn in files:
         g = np.load(os.path.join(GOLDEN, fn))
-        y, cons, prod = oracle.fir(int(g["dtype"]), bool(g["taps_complex"]), g["taps"], int(g["M"]), int(g["L"]), g["x"])
+        args = (int(g["dtype"]), bool(g["taps_complex"]), g["taps"], int(g["M"]), int(g["L"]))
+        y, cons, prod = oracle.fir(*args, g["x"])
         assert cons == int(g["consumed"]) and prod == int(g["produced"]), fn
         assert np.array_equal(y.view(np.uint8), g["y"].view(np.uint8)), fn
+        yb, cb, pb = oracle.fir(*args, g["x"][:500], zero_tail=True)
+        assert cb == int(g["burst_consumed"]) and pb == int(g["burst_produced"]), fn
+        assert np.array_equal(yb.view(np.uint8), g["burst_y"].view(np.uint8)), fn
         assert str(g["source"]) == "reference:filter/FIRFilter.cpp", fn
 
 
