@@ -136,6 +136,37 @@ int b200c_fir_bank_run(b200c_fir_bank *b, const void *d_in, size_t in_stride, si
                        size_t out_stride, size_t out_capacity, int zero_tail, size_t *consumed, size_t *produced,
                        void *stream);
 
+/* ------------------------------------- polyphase filter-bank channelizer (one stream in) --- */
+/* Splits ONE wideband complex float32 stream into `nchan` = M baseband channels, decimated by `decim` = D.
+ * Channel c is exactly /comms/fir_filter with REAL taps h, decimation D (filter/FIRFilter.cpp:278-302: it
+ * emits on the last of every D inputs) applied to the stream mixed down by c/M cycles per sample:
+ *   z[i] = x[i] exp(-2 pi i c (s + i) / M),     s = stream_index = absolute stream index of d_in[0]
+ * i.e., with m_t = (ntaps-1) + t D + (D-1) the newest input sample of output frame t,
+ *   y_c[t] = sum_{n < ntaps} h[n] x[m_t - n] exp(-2 pi i c (s + m_t - n) / M).
+ * Channel c is centred at +c/M cycles per sample; channels c >= M/2 are the negative frequencies.  Only
+ * s mod M matters, so a stream cut into pieces (or segments on several GPUs) keeps its channel phases as long as
+ * each call passes the absolute index of its first element.
+ * Computed as a polyphase filter bank: ceil(ntaps/M) real-tap products per branch and frame, then one M-point
+ * FFT per frame; each input sample is read about once and each output written once.
+ *
+ * dtype B200C_CF32 only, M a power of two in [2, 4096] (else B200C_ERR_UNSUPPORTED); D >= 1 dividing M (D = M:
+ * critically sampled, D = M/2: 2x oversampled) and 1 <= ntaps <= 16 M (else B200C_ERR_INVALID).  Create-time
+ * arguments are checked before any device call.  Taps: real doubles stored as float32, {1} after create. */
+typedef struct b200c_chan b200c_chan;
+int b200c_chan_create(b200c_chan **out, int dtype, size_t nchan, size_t decim, int device);
+int b200c_chan_destroy(b200c_chan *h);
+int b200c_chan_set_taps(b200c_chan *h, const double *taps, size_t ntaps);
+/* input_require = ntaps - 1 + decim */
+int b200c_chan_info(const b200c_chan *h, size_t *nchan, size_t *decim, size_t *ntaps, size_t *input_require);
+/* d_in: in_elems complex float32 samples on the device, the first ntaps-1 of them history (as b200c_fir_run with
+ * K = ntaps, L = 1).  F = min((in_elems - (ntaps-1)) / D, out_capacity), 0 when in_elems < ntaps-1+D;
+ * *consumed = F D, *produced = F.  Frame t of channel c goes to d_out[c * out_stride + t] (elements): the layout
+ * b200c_fir_bank_run reads, so the channels can be post-filtered by a bank without a copy.  Nothing else of d_out
+ * is written.  Null buffers (with F > 0) or out_stride < F -> B200C_ERR_INVALID.  Stateless, asynchronous on
+ * `stream`, one kernel launch; a frame's value does not depend on how the stream was cut into calls (bit for bit). */
+int b200c_chan_run(b200c_chan *h, const void *d_in, size_t in_elems, uint64_t stream_index, void *d_out, size_t out_stride,
+                   size_t out_capacity, size_t *consumed, size_t *produced, void *stream);
+
 /* ------------------------------------------------------------------------- /comms/fft --- */
 typedef struct b200c_fft b200c_fft;
 

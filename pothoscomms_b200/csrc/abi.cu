@@ -10,6 +10,7 @@
 #include <string>
 #include <vector>
 
+#include "chan.hpp"
 #include "common.hpp"
 #include "fir_imma.hpp"
 #include "fft.hpp"
@@ -139,6 +140,12 @@ struct b200c_fir_bank {
     void *d_hf_all = nullptr;      // [nchan][N] tap spectra gathered for the one-launch path
     size_t hf_capacity = 0;
     bool dirty = true;
+};
+
+struct b200c_chan {
+    int device = 0;
+    DevInfo di;
+    ChanPlan plan;
 };
 
 struct b200c_fft {
@@ -568,6 +575,83 @@ int b200c_fir_bank_run(b200c_fir_bank *b, const void *d_in, size_t in_stride, si
         if (rc) return rc;
     }
     return B200C_OK;
+}
+
+/* ------------------------------------------------------------------- channelizer --- */
+int b200c_chan_create(b200c_chan **out, int dtype, size_t nchan, size_t decim, int device)
+{
+    if (!out) return B200C_ERR_INVALID;
+    *out = nullptr;
+    if (dtype != B200C_CF32) { set_error("channelizer: dtype %d unsupported (complex float32 only)", dtype); return B200C_ERR_UNSUPPORTED; }
+    if (nchan < 2 || nchan > kChanMaxChannels || (nchan & (nchan - 1))) {
+        set_error("channelizer: %zu channels unsupported (a power of two from 2 to %zu)", nchan, kChanMaxChannels);
+        return B200C_ERR_UNSUPPORTED;
+    }
+    if (decim == 0 || nchan % decim) { set_error("channelizer: decimation %zu must divide the channel count %zu", decim, nchan); return B200C_ERR_INVALID; }
+    DevInfo di;
+    int rc = dev_info(device, di);
+    if (rc) return rc;
+    b200c_chan *h = new (std::nothrow) b200c_chan();
+    if (!h) { set_error("out of host memory"); return B200C_ERR_NOMEM; }
+    h->device = device; h->di = di;
+    DeviceGuard g(device);
+    if (!g.ok) { delete h; set_error("cudaSetDevice(%d) failed", device); return B200C_ERR_CUDA; }
+    rc = chan_plan_create(h->plan, nchan, decim, di.smem_optin);
+    const double one = 1.0;   // taps {1}, as FIRFilter() (filter/FIRFilter.cpp:125)
+    if (!rc) rc = chan_set_taps(h->plan, &one, 1);
+    if (rc) { b200c_chan_destroy(h); return rc; }
+    *out = h;
+    return B200C_OK;
+}
+
+int b200c_chan_destroy(b200c_chan *h)
+{
+    if (!h) return B200C_OK;
+    {
+        DeviceGuard g(h->device);
+        chan_plan_destroy(h->plan);
+    }
+    delete h;
+    return B200C_OK;
+}
+
+int b200c_chan_set_taps(b200c_chan *h, const double *taps, size_t ntaps)
+{
+    if (!h) return B200C_ERR_INVALID;
+    if (ntaps == 0 || !taps) { set_error("channelizer: taps cannot be empty"); return B200C_ERR_INVALID; }
+    if (ntaps > kChanMaxTapsPerBranch * (size_t)h->plan.M) {
+        set_error("channelizer: %zu taps exceed 16 per branch (%zu for %d channels)", ntaps, kChanMaxTapsPerBranch * (size_t)h->plan.M, h->plan.M);
+        return B200C_ERR_INVALID;
+    }
+    DeviceGuard g(h->device);
+    if (!g.ok) { set_error("cudaSetDevice(%d) failed", h->device); return B200C_ERR_CUDA; }
+    return chan_set_taps(h->plan, taps, ntaps);
+}
+
+int b200c_chan_info(const b200c_chan *h, size_t *nchan, size_t *decim, size_t *ntaps, size_t *input_require)
+{
+    if (!h) return B200C_ERR_INVALID;
+    if (nchan) *nchan = (size_t)h->plan.M;
+    if (decim) *decim = (size_t)h->plan.D;
+    if (ntaps) *ntaps = h->plan.ntaps;
+    if (input_require) *input_require = h->plan.ntaps - 1 + (size_t)h->plan.D;
+    return B200C_OK;
+}
+
+int b200c_chan_run(b200c_chan *h, const void *d_in, size_t in_elems, uint64_t stream_index, void *d_out, size_t out_stride,
+                   size_t out_capacity, size_t *consumed, size_t *produced, void *stream)
+{
+    if (!h) return B200C_ERR_INVALID;
+    const size_t Km1 = h->plan.ntaps - 1, D = (size_t)h->plan.D;
+    const size_t F = in_elems >= Km1 + D ? std::min((in_elems - Km1) / D, out_capacity) : 0;
+    if (consumed) *consumed = F * D;
+    if (produced) *produced = F;
+    if (F == 0) return B200C_OK;
+    if (!d_in || !d_out) { set_error("b200c_chan_run: null device buffer"); return B200C_ERR_INVALID; }
+    if (out_stride < F) { set_error("channelizer: output stride %zu shorter than the %zu frames produced", out_stride, F); return B200C_ERR_INVALID; }
+    DeviceGuard g(h->device);
+    if (!g.ok) { set_error("cudaSetDevice(%d) failed", h->device); return B200C_ERR_CUDA; }
+    return chan_launch(h->plan, d_in, F, stream_index, d_out, out_stride, (cudaStream_t)stream);
 }
 
 /* ----------------------------------------------------------------------------- FFT --- */

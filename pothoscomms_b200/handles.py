@@ -196,6 +196,57 @@ class FirFilterBank:
         return c.value, p.value
 
 
+class Channelizer:
+    """Owner of a b200c_chan handle: one complex float32 stream into `nchan` baseband channels (polyphase
+    filter bank), decimated by `decim`.  Channel c is /comms/fir_filter with the real prototype taps applied to
+    the stream mixed down by c/nchan cycles per sample (include/b200comms.h has the exact definition)."""
+
+    def __init__(self, dtype, nchan: int, decim: int, device: int = 0):
+        self.dtype = dtype_code(dtype)
+        self.nchan = int(nchan)
+        self.decim = int(decim)
+        self.device = device
+        self._h = ctypes.c_void_p()
+        if self.nchan < 0 or self.decim < 0:
+            raise _abi.InvalidArgumentError(_abi.ERR_INVALID, "negative channel count or decimation")
+        _abi.check(_abi.lib().b200c_chan_create(ctypes.byref(self._h), self.dtype, self.nchan, self.decim, device))
+
+    def close(self):
+        try:
+            if getattr(self, "_h", None) is not None and self._h:
+                _abi.lib().b200c_chan_destroy(self._h)
+                self._h = ctypes.c_void_p()
+        except (TypeError, AttributeError):
+            pass
+
+    __del__ = close
+
+    def set_taps(self, taps):
+        t = _taps_array(taps, False)
+        _abi.check(_abi.lib().b200c_chan_set_taps(self._h, t.ctypes.data, t.size))
+
+    def info(self):
+        """(nchan, decim, ntaps, input_require)"""
+        n, d, k, req = (ctypes.c_size_t() for _ in range(4))
+        _abi.check(_abi.lib().b200c_chan_info(self._h, ctypes.byref(n), ctypes.byref(d), ctypes.byref(k), ctypes.byref(req)))
+        return n.value, d.value, k.value, req.value
+
+    def run(self, d_in, out, stream_index: int = 0, out_capacity: int | None = None, stream=None):
+        """d_in: CUDA tensor [n, 2] float32 (ntaps-1 history samples first); out: CUDA tensor [nchan, capacity, 2]
+        float32, frame t of channel c lands in out[c, t].  stream_index: absolute stream index of d_in[0].
+        Returns (consumed, produced)."""
+        import torch
+        assert d_in.is_cuda and d_in.is_contiguous() and d_in.dtype == torch.float32
+        assert out.is_cuda and out.is_contiguous() and out.dtype == torch.float32 and out.dim() == 3 and out.shape[0] == self.nchan
+        stride = out.shape[1]
+        cap = stride if out_capacity is None else int(out_capacity)
+        c, p = ctypes.c_size_t(), ctypes.c_size_t()
+        _abi.check(_abi.lib().b200c_chan_run(self._h, ctypes.c_void_p(d_in.data_ptr()), d_in.numel() // 2,
+                                             int(stream_index) & (2**64 - 1), ctypes.c_void_p(out.data_ptr()), stride, cap,
+                                             ctypes.byref(c), ctypes.byref(p), _stream_ptr(stream, d_in.device)))
+        return c.value, p.value
+
+
 class Fft:
     """Owner of a b200c_fft handle (the FFTAux of one /comms/fft block)."""
 
