@@ -167,6 +167,39 @@ int b200c_chan_info(const b200c_chan *h, size_t *nchan, size_t *decim, size_t *n
 int b200c_chan_run(b200c_chan *h, const void *d_in, size_t in_elems, uint64_t stream_index, void *d_out, size_t out_stride,
                    size_t out_capacity, size_t *consumed, size_t *produced, void *stream);
 
+/* --------------------------------- polyphase synthesis filter bank (one stream out) --- */
+/* The transpose of the channelizer: puts `nchan` = M baseband channels, interpolated by `interp` = D, back into
+ * ONE wideband complex float32 stream.  Channel c goes through /comms/fir_filter with REAL taps g, interpolation
+ * D and decimation 1, is mixed up by +c/M cycles per sample, and all channels are summed.  With K = ceil(ntaps/D)
+ * and s = stream_index, the absolute stream index of d_out[0], output sample m = t D + j (j < D) is
+ *   y[t D + j] = sum_{c < M} exp(+2 pi i c (s + t D + j) / M) sum_{k < K, j + k D < ntaps} g[j + k D] X_c[K-1 + t - k]
+ * Channels c >= M/2 are the negative frequencies (the channelizer's convention).  Only s mod M matters.
+ * Computed as a polyphase synthesizer: one inverse M-point FFT per input frame, then K real-tap products per
+ * output sample; each input frame is read about once and each output sample written once.
+ *
+ * dtype B200C_CF32 only, M a power of two in [2, 4096] (else B200C_ERR_UNSUPPORTED); D >= 1 dividing M (D = M:
+ * critically sampled, D = M/2: 2x oversampled) and 1 <= ntaps <= min(16 M, 32 D), so K <= 32 (else
+ * B200C_ERR_INVALID; a refused set_taps keeps the old taps).  Create-time arguments are checked before any device
+ * call.  Taps: real doubles stored as float32, {1} after create.
+ *
+ * Perfect reconstruction after b200c_chan with D = M/2 (INTEGRATION §1): analysis h = firwin(12M+1, 1/M,
+ * kaiser 10), synthesis g = D firwin(28D+1, 2/M, kaiser_beta(90)); synthesizer stream_index
+ * s_a + (ntaps_h - 1) + (D - 1) + (K_g - 1) D, where s_a is the channelizer's. */
+typedef struct b200c_synth b200c_synth;
+int b200c_synth_create(b200c_synth **out, int dtype, size_t nchan, size_t interp, int device);
+int b200c_synth_destroy(b200c_synth *h);
+int b200c_synth_set_taps(b200c_synth *h, const double *taps, size_t ntaps);
+/* input_require = K frames per channel */
+int b200c_synth_info(const b200c_synth *h, size_t *nchan, size_t *interp, size_t *ntaps, size_t *input_require);
+/* d_in: M channel rows in the channelizer's output layout, frame i of channel c at d_in[c * in_stride + i] for
+ * i < in_frames; the first K-1 frames of every channel are history (as b200c_fir_run with L = D, M = 1).
+ * F = min(in_frames - (K-1), out_capacity / D), 0 when in_frames < K; *consumed = F frames per channel,
+ * *produced = F D samples, written to d_out[0 .. F D) and nowhere else.  Null buffers (with F > 0) or
+ * in_stride < in_frames -> B200C_ERR_INVALID.  Stateless, asynchronous on `stream`, one kernel launch; an output
+ * sample's value does not depend on how the stream was cut into calls (bit for bit). */
+int b200c_synth_run(b200c_synth *h, const void *d_in, size_t in_stride, size_t in_frames, uint64_t stream_index, void *d_out,
+                    size_t out_capacity, size_t *consumed, size_t *produced, void *stream);
+
 /* ------------------------------------------------------------------------- /comms/fft --- */
 typedef struct b200c_fft b200c_fft;
 

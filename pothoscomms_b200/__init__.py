@@ -15,6 +15,6 @@ from ._abi import B200CommsError, InvalidArgumentError
 
 _abi.lib()  # fail loudly at import time if the CUDA library is not built
 
-from .handles import Channelizer, DeviceRing, Fft, FirFilter, FirFilterBank  # noqa: E402
+from .handles import Channelizer, DeviceRing, Fft, FirFilter, FirFilterBank, Synthesizer  # noqa: E402
 
-__all__ = ["FirFilter", "FirFilterBank", "Channelizer", "Fft", "DeviceRing", "B200CommsError", "InvalidArgumentError"]
+__all__ = ["FirFilter", "FirFilterBank", "Channelizer", "Synthesizer", "Fft", "DeviceRing", "B200CommsError", "InvalidArgumentError"]

@@ -15,6 +15,7 @@
 #include "fir_imma.hpp"
 #include "fft.hpp"
 #include "fir.hpp"
+#include "synth.hpp"
 
 namespace b200c {
 
@@ -146,6 +147,12 @@ struct b200c_chan {
     int device = 0;
     DevInfo di;
     ChanPlan plan;
+};
+
+struct b200c_synth {
+    int device = 0;
+    DevInfo di;
+    SynthPlan plan;
 };
 
 struct b200c_fft {
@@ -652,6 +659,87 @@ int b200c_chan_run(b200c_chan *h, const void *d_in, size_t in_elems, uint64_t st
     DeviceGuard g(h->device);
     if (!g.ok) { set_error("cudaSetDevice(%d) failed", h->device); return B200C_ERR_CUDA; }
     return chan_launch(h->plan, d_in, F, stream_index, d_out, out_stride, (cudaStream_t)stream);
+}
+
+/* ------------------------------------------------------------------- synthesizer --- */
+int b200c_synth_create(b200c_synth **out, int dtype, size_t nchan, size_t interp, int device)
+{
+    if (!out) return B200C_ERR_INVALID;
+    *out = nullptr;
+    if (dtype != B200C_CF32) { set_error("synthesizer: dtype %d unsupported (complex float32 only)", dtype); return B200C_ERR_UNSUPPORTED; }
+    if (nchan < 2 || nchan > kSynthMaxChannels || (nchan & (nchan - 1))) {
+        set_error("synthesizer: %zu channels unsupported (a power of two from 2 to %zu)", nchan, kSynthMaxChannels);
+        return B200C_ERR_UNSUPPORTED;
+    }
+    if (interp == 0 || nchan % interp) { set_error("synthesizer: interpolation %zu must divide the channel count %zu", interp, nchan); return B200C_ERR_INVALID; }
+    DevInfo di;
+    int rc = dev_info(device, di);
+    if (rc) return rc;
+    b200c_synth *h = new (std::nothrow) b200c_synth();
+    if (!h) { set_error("out of host memory"); return B200C_ERR_NOMEM; }
+    h->device = device; h->di = di;
+    DeviceGuard g(device);
+    if (!g.ok) { delete h; set_error("cudaSetDevice(%d) failed", device); return B200C_ERR_CUDA; }
+    rc = synth_plan_create(h->plan, nchan, interp, di.smem_optin);
+    const double one = 1.0;   // taps {1}, as FIRFilter() (filter/FIRFilter.cpp:125)
+    if (!rc) rc = synth_set_taps(h->plan, &one, 1);
+    if (rc) { b200c_synth_destroy(h); return rc; }
+    *out = h;
+    return B200C_OK;
+}
+
+int b200c_synth_destroy(b200c_synth *h)
+{
+    if (!h) return B200C_OK;
+    {
+        DeviceGuard g(h->device);
+        synth_plan_destroy(h->plan);
+    }
+    delete h;
+    return B200C_OK;
+}
+
+int b200c_synth_set_taps(b200c_synth *h, const double *taps, size_t ntaps)
+{
+    if (!h) return B200C_ERR_INVALID;
+    if (ntaps == 0 || !taps) { set_error("synthesizer: taps cannot be empty"); return B200C_ERR_INVALID; }
+    const size_t M = (size_t)h->plan.M, D = (size_t)h->plan.D;
+    const size_t limit = std::min(kSynthMaxTapsPerChannel * M, kSynthMaxTapsPerPhase * D);
+    if (ntaps > limit) {
+        set_error("synthesizer: %zu taps exceed min(16 M, 32 D) = %zu for %zu channels, interpolation %zu", ntaps, limit, M, D);
+        return B200C_ERR_INVALID;
+    }
+    DeviceGuard g(h->device);
+    if (!g.ok) { set_error("cudaSetDevice(%d) failed", h->device); return B200C_ERR_CUDA; }
+    return synth_set_taps(h->plan, taps, ntaps);
+}
+
+int b200c_synth_info(const b200c_synth *h, size_t *nchan, size_t *interp, size_t *ntaps, size_t *input_require)
+{
+    if (!h) return B200C_ERR_INVALID;
+    if (nchan) *nchan = (size_t)h->plan.M;
+    if (interp) *interp = (size_t)h->plan.D;
+    if (ntaps) *ntaps = h->plan.ntaps;
+    if (input_require) *input_require = (size_t)h->plan.K;
+    return B200C_OK;
+}
+
+int b200c_synth_run(b200c_synth *h, const void *d_in, size_t in_stride, size_t in_frames, uint64_t stream_index, void *d_out,
+                    size_t out_capacity, size_t *consumed, size_t *produced, void *stream)
+{
+    if (!h) return B200C_ERR_INVALID;
+    if (consumed) *consumed = 0;
+    if (produced) *produced = 0;
+    if (in_stride < in_frames) { set_error("synthesizer: input stride %zu shorter than the %zu frames given", in_stride, in_frames); return B200C_ERR_INVALID; }
+    const size_t Km1 = (size_t)h->plan.K - 1, D = (size_t)h->plan.D;
+    const size_t F = in_frames > Km1 ? std::min(in_frames - Km1, out_capacity / D) : 0;
+    if (consumed) *consumed = F;
+    if (produced) *produced = F * D;
+    if (F == 0) return B200C_OK;
+    if (!d_in || !d_out) { set_error("b200c_synth_run: null device buffer"); return B200C_ERR_INVALID; }
+    DeviceGuard g(h->device);
+    if (!g.ok) { set_error("cudaSetDevice(%d) failed", h->device); return B200C_ERR_CUDA; }
+    return synth_launch(h->plan, d_in, in_stride, F, stream_index, d_out, (cudaStream_t)stream);
 }
 
 /* ----------------------------------------------------------------------------- FFT --- */

@@ -247,6 +247,61 @@ class Channelizer:
         return c.value, p.value
 
 
+class Synthesizer:
+    """Owner of a b200c_synth handle: `nchan` baseband channels, interpolated by `interp`, back into one complex
+    float32 stream (polyphase synthesis filter bank, the transpose of Channelizer).  Channel c is /comms/fir_filter
+    with the real prototype taps and interpolation `interp`, mixed up by +c/nchan cycles per sample, and the channels
+    are summed (include/b200comms.h has the exact definition)."""
+
+    def __init__(self, dtype, nchan: int, interp: int, device: int = 0):
+        self.dtype = dtype_code(dtype)
+        self.nchan = int(nchan)
+        self.interp = int(interp)
+        self.device = device
+        self._h = ctypes.c_void_p()
+        if self.nchan < 0 or self.interp < 0:
+            raise _abi.InvalidArgumentError(_abi.ERR_INVALID, "negative channel count or interpolation")
+        _abi.check(_abi.lib().b200c_synth_create(ctypes.byref(self._h), self.dtype, self.nchan, self.interp, device))
+
+    def close(self):
+        try:
+            if getattr(self, "_h", None) is not None and self._h:
+                _abi.lib().b200c_synth_destroy(self._h)
+                self._h = ctypes.c_void_p()
+        except (TypeError, AttributeError):
+            pass
+
+    __del__ = close
+
+    def set_taps(self, taps):
+        t = _taps_array(taps, False)
+        _abi.check(_abi.lib().b200c_synth_set_taps(self._h, t.ctypes.data, t.size))
+
+    def info(self):
+        """(nchan, interp, ntaps, input_require), input_require = ceil(ntaps / interp) frames"""
+        n, d, k, req = (ctypes.c_size_t() for _ in range(4))
+        _abi.check(_abi.lib().b200c_synth_info(self._h, ctypes.byref(n), ctypes.byref(d), ctypes.byref(k), ctypes.byref(req)))
+        return n.value, d.value, k.value, req.value
+
+    def run(self, d_in, out, stream_index: int = 0, in_frames: int | None = None, out_capacity: int | None = None,
+            stream=None):
+        """d_in: CUDA tensor [nchan, stride, 2] float32, frame i of channel c in d_in[c, i] (the Channelizer's output
+        layout; the first ceil(ntaps/interp)-1 frames are history); out: CUDA tensor [n, 2] float32.
+        stream_index: absolute stream index of out[0].  Returns (consumed frames per channel, produced samples)."""
+        import torch
+        assert d_in.is_cuda and d_in.is_contiguous() and d_in.dtype == torch.float32
+        assert d_in.dim() == 3 and d_in.shape[0] == self.nchan
+        assert out.is_cuda and out.is_contiguous() and out.dtype == torch.float32
+        stride = d_in.shape[1]
+        frames = stride if in_frames is None else int(in_frames)
+        cap = out.numel() // 2 if out_capacity is None else int(out_capacity)
+        c, p = ctypes.c_size_t(), ctypes.c_size_t()
+        _abi.check(_abi.lib().b200c_synth_run(self._h, ctypes.c_void_p(d_in.data_ptr()), stride, frames,
+                                              int(stream_index) & (2**64 - 1), ctypes.c_void_p(out.data_ptr()), cap,
+                                              ctypes.byref(c), ctypes.byref(p), _stream_ptr(stream, d_in.device)))
+        return c.value, p.value
+
+
 class Fft:
     """Owner of a b200c_fft handle (the FFTAux of one /comms/fft block)."""
 
