@@ -124,8 +124,8 @@ int b200c_fir_run_host(b200c_fir *h, const void *h_in, size_t in_elems, void *h_
  * driven together: channel c reads d_in + c*in_stride and writes d_out + c*out_stride (strides in
  * elements), all channels see the same in_elems / out_capacity, so consume / produce are common.
  * Every channel has its own taps (b200c_fir_bank_set_taps) but the same tap COUNT and rates.
- * complex float32 streams run as ONE launch over (channel, block); other types run the
- * channels' kernels back to back on `stream`.  Results per channel are exactly b200c_fir_run's. */
+ * complex float32 streams at L = M = 1 run as ONE launch over (channel, block); other types and
+ * rates run the channels' kernels back to back on `stream`.  Results per channel are b200c_fir_run's. */
 typedef struct b200c_fir_bank b200c_fir_bank;
 int b200c_fir_bank_create(b200c_fir_bank **out, int dtype, int taps_kind, size_t nchan, int device);
 int b200c_fir_bank_destroy(b200c_fir_bank *b);

@@ -549,8 +549,9 @@ int b200c_fir_bank_run(b200c_fir_bank *b, const void *d_in, size_t in_stride, si
     if (nch > 1 && (in_stride < in_elems || out_stride < p)) { set_error("filter bank: channel stride shorter than the channel"); return B200C_ERR_INVALID; }
     DeviceGuard g(b->device);
     if (!g.ok) { set_error("cudaSetDevice(%d) failed", b->device); return B200C_ERR_CUDA; }
-    bool fast = h0->use_os && !h0->os.general && !h0->os.real32;   // one launch over (channel, block): complex float32, L = M = 1
-    for (auto *ch : b->ch) fast = fast && ch->use_os && !ch->os.general && !ch->os.real32 && ch->os.N == h0->os.N;
+    // one launch over (channel, block) where every channel's plan allows it (fir_os_batchable: complex float32, L = M = 1)
+    bool fast = true;
+    for (auto *ch : b->ch) fast = fast && ch->use_os && fir_os_batchable(ch->os) && ch->os.N == h0->os.N;
     if (fast) {
         // one launch over (channel, block): gather the channels' tap spectra once per setTaps()
         const size_t N = (size_t)h0->os.N, row = N * 2 * sizeof(float);

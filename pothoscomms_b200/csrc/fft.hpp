@@ -106,6 +106,9 @@ struct FirOsBatch {
     long long in_stride = 0, out_stride = 0;
     const void *d_hf = nullptr;
 };
+// Whether one batched launch can serve a bank whose channels all have this plan: complex float32, L = M = 1, a
+// 1024- or 4096-point tap spectrum (d_hf1k / d_hf).  Every other plan runs channel by channel.
+bool fir_os_batchable(const FirOsPlan &p);
 // nq = output blocks q (= consumed / M); outputs written = nq * L
 int fir_os_launch(const FirOsPlan &p, const void *d_in, size_t in_elems, void *d_out, size_t nq, int sm_count,
                   cudaStream_t stream, const FirOsBatch *batch = nullptr);

@@ -171,7 +171,7 @@ __global__ void __launch_bounds__(64, MINB) fir_os64_kernel(const FirOs64Args a)
 //     blocks part*4 + g, + parts*4, ... for the four groups g -- so the spectrum is staged once per task (once per
 //     channel when parts = 1) and the 64 loads per thread and block become LDS; ncu had the global loads as the
 //     long_scoreboard / lg_throttle stalls of the one-transform-per-CTA kernel (profiles/r02j_prof_os64p_c5.txt).
-// The host picks `parts` so that nchan * parts tasks fill whole rounds of CTAs: 1 for a 1024-channel bank, 15 for the
+// The host picks `parts` so that nchan * parts tasks fill whole rounds of CTAs: 1 for a 1024-channel bank, 8 for the
 // 128 channels one of 8 GPUs holds, gridDim.x for a single stream (every CTA one task, the spectrum staged once).
 constexpr int kOs64Groups = 4;
 __global__ void __launch_bounds__(64 * kOs64Groups, 1) fir_os64p_kernel(const FirOs64Args a)
@@ -1562,13 +1562,15 @@ static cudaError_t launch_dependent(Kernel kern, int grid, int block, size_t sme
     return cudaLaunchKernelEx(&cfg, kern, a);
 }
 
+bool fir_os_batchable(const FirOsPlan &p) { return p.ready && !p.x32 && !p.general && !p.real32; }
+
 int fir_os_launch(const FirOsPlan &p, const void *d_in, size_t in_elems, void *d_out, size_t nq, int sm_count,
                   cudaStream_t stream, const FirOsBatch *batch)
 {
     if (nq == 0) return B200C_OK;
+    if (batch && !fir_os_batchable(p)) { set_error("filter bank: the batched launch serves complex float32 L = M = 1 only"); return B200C_ERR_UNSUPPORTED; }
     const int nchan = batch ? batch->nchan : 1;
     if (p.x32) {
-        if (batch) { set_error("filter bank: the batched launch serves complex float32 L = M = 1 only"); return B200C_ERR_UNSUPPORTED; }
         FirOsX32Args a;
         a.in = d_in; a.out = d_out; a.hx = p.d_hx; a.tw = p.d_tw1k; a.tw3 = p.d_tw3;
         a.n_in = (long long)in_elems; a.n_out = (long long)nq * 3; a.p0 = p.p0; a.m0 = p.m0;
@@ -1595,7 +1597,6 @@ int fir_os_launch(const FirOsPlan &p, const void *d_in, size_t in_elems, void *d
         return B200C_OK;
     }
     if (p.general) {
-        if (batch) { set_error("filter bank: the batched launch serves complex float32 L = M = 1 only"); return B200C_ERR_UNSUPPORTED; }
         FirOs32GArgs a;
         a.in = d_in; a.out = d_out; a.H = p.d_H; a.tw = p.d_tw1k;
         a.n_in = (long long)in_elems; a.nq = (long long)nq; a.start0 = p.start0; a.L = p.L; a.hop = p.hopq;
@@ -1627,7 +1628,6 @@ int fir_os_launch(const FirOsPlan &p, const void *d_in, size_t in_elems, void *d
 #undef OSG
     }
     if (p.real32) {
-        if (batch) { set_error("filter bank: the batched launch serves complex float32 L = M = 1 only"); return B200C_ERR_UNSUPPORTED; }
         FirOs32RArgs a;
         a.in = static_cast<const float *>(d_in); a.out = static_cast<float *>(d_out); a.hf = p.d_hf1k; a.tw = p.d_tw1k;
         a.n_in = (long long)in_elems; a.n_out = (long long)nq; a.K = p.K;
