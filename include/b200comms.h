@@ -167,6 +167,37 @@ int b200c_chan_info(const b200c_chan *h, size_t *nchan, size_t *decim, size_t *n
 int b200c_chan_run(b200c_chan *h, const void *d_in, size_t in_elems, uint64_t stream_index, void *d_out, size_t out_stride,
                    size_t out_capacity, size_t *consumed, size_t *produced, void *stream);
 
+/* --------------------------- real-input polyphase filter-bank channelizer (one real stream in) --- */
+/* The channelizer above applied to ONE real stream x of float32 or int16 (what direct-IF / direct-RF sampling
+ * digitizers deliver), keeping only the channels that are not complex-conjugate mirrors.  With M = branches, D =
+ * decim, s = stream_index (the absolute index of d_in[0]) and m_t = (ntaps-1) + t D + (D-1), for c = 0 .. M/2
+ *   y_c[t] = sum_{n < ntaps} h[n] x[m_t - n] exp(-2 pi i c (s + m_t - n) / M).
+ * Channel c is centred at +c/M cycles per sample; the channels M/2 < c < M of the complex definition are
+ * conj(y_{M-c}) and are not produced.  Channels 0 and M/2 are real: their imaginary parts are written as exactly 0.
+ * Only s mod M matters.  int16 samples are converted to float32 exactly (no scaling), so int16 input gives output
+ * bit-identical to float32 input of the same values.
+ * Computed as a polyphase filter bank: ceil(ntaps/M) real products per branch and frame, the real M-point frame
+ * packed into one M/2-point complex FFT (within the frame, never two frames together), then the even/odd split.
+ *
+ * dtype B200C_F32 or B200C_I16 (else B200C_ERR_UNSUPPORTED); M a power of two in [2, 8192] (else
+ * B200C_ERR_UNSUPPORTED); D >= 1 dividing M (else B200C_ERR_INVALID).  Checked before any device call.  Taps: real
+ * doubles stored as float32, {1} after create; 1 <= ntaps <= 16 M, else B200C_ERR_INVALID and the old taps stay. */
+typedef struct b200c_rchan b200c_rchan;
+int b200c_rchan_create(b200c_rchan **out, int dtype, size_t m, size_t decim, int device);
+int b200c_rchan_destroy(b200c_rchan *h);
+int b200c_rchan_set_taps(b200c_rchan *h, const double *taps, size_t ntaps);
+/* nchan = M/2 + 1 output rows; input_require = ntaps - 1 + decim */
+int b200c_rchan_info(const b200c_rchan *h, size_t *m, size_t *nchan, size_t *decim, size_t *ntaps, size_t *input_require);
+/* d_in: in_elems real samples of the handle's dtype on the device, the first ntaps-1 of them history; it may start
+ * at any element offset.  F = min((in_elems - (ntaps-1)) / D, out_capacity), 0 when in_elems < ntaps-1+D;
+ * *consumed = F D, *produced = F.  Frame t of channel c (c <= M/2) goes to d_out[c * out_stride + t] (complex
+ * float32 elements): the layout b200c_fir_bank_run reads, so a complex float32 bank of M/2 + 1 channels can
+ * post-filter them without a copy.  Nothing else of d_out is written.  Null buffers (with F > 0) or out_stride < F
+ * -> B200C_ERR_INVALID.  Stateless, asynchronous on `stream`, one kernel launch; a frame's value does not depend on
+ * how the stream was cut into calls (bit for bit). */
+int b200c_rchan_run(b200c_rchan *h, const void *d_in, size_t in_elems, uint64_t stream_index, void *d_out,
+                    size_t out_stride, size_t out_capacity, size_t *consumed, size_t *produced, void *stream);
+
 /* --------------------------------- polyphase synthesis filter bank (one stream out) --- */
 /* The transpose of the channelizer: puts `nchan` = M baseband channels, interpolated by `interp` = D, back into
  * ONE wideband complex float32 stream.  Channel c goes through /comms/fir_filter with REAL taps g, interpolation

@@ -56,6 +56,12 @@ SYMBOLS = {
     "b200c_chan_info": (_i, [_vp, _psz, _psz, _psz, _psz]),
     # stream_index is a uint64: a default int conversion would cut it to 32 bits
     "b200c_chan_run": (_i, [_vp, _vp, _sz, ctypes.c_uint64, _vp, _sz, _sz, _psz, _psz, _vp]),
+    "b200c_rchan_create": (_i, [_pvp, _i, _sz, _sz, _i]),
+    "b200c_rchan_destroy": (_i, [_vp]),
+    "b200c_rchan_set_taps": (_i, [_vp, _vp, _sz]),
+    "b200c_rchan_info": (_i, [_vp, _psz, _psz, _psz, _psz, _psz]),
+    # stream_index is a uint64, as for b200c_chan_run
+    "b200c_rchan_run": (_i, [_vp, _vp, _sz, ctypes.c_uint64, _vp, _sz, _sz, _psz, _psz, _vp]),
     "b200c_synth_create": (_i, [_pvp, _i, _sz, _sz, _i]),
     "b200c_synth_destroy": (_i, [_vp]),
     "b200c_synth_set_taps": (_i, [_vp, _vp, _sz]),

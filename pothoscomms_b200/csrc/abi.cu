@@ -15,6 +15,7 @@
 #include "fir_imma.hpp"
 #include "fft.hpp"
 #include "fir.hpp"
+#include "rchan.hpp"
 #include "synth.hpp"
 
 namespace b200c {
@@ -145,6 +146,13 @@ struct b200c_fir_bank {
 
 struct b200c_chan {
     int device = 0;
+    DevInfo di;
+    ChanPlan plan;
+};
+
+struct b200c_rchan {
+    int device = 0;
+    int dtype = B200C_F32;
     DevInfo di;
     ChanPlan plan;
 };
@@ -660,6 +668,87 @@ int b200c_chan_run(b200c_chan *h, const void *d_in, size_t in_elems, uint64_t st
     DeviceGuard g(h->device);
     if (!g.ok) { set_error("cudaSetDevice(%d) failed", h->device); return B200C_ERR_CUDA; }
     return chan_launch(h->plan, d_in, F, stream_index, d_out, out_stride, (cudaStream_t)stream);
+}
+
+/* -------------------------------------------------------- real-input channelizer --- */
+int b200c_rchan_create(b200c_rchan **out, int dtype, size_t m, size_t decim, int device)
+{
+    if (!out) return B200C_ERR_INVALID;
+    *out = nullptr;
+    if (dtype != B200C_F32 && dtype != B200C_I16) {
+        set_error("real channelizer: dtype %d unsupported (float32 or int16 only)", dtype);
+        return B200C_ERR_UNSUPPORTED;
+    }
+    if (m < 2 || m > kRChanMaxBranches || (m & (m - 1))) {
+        set_error("real channelizer: %zu branches unsupported (a power of two from 2 to %zu)", m, kRChanMaxBranches);
+        return B200C_ERR_UNSUPPORTED;
+    }
+    if (decim == 0 || m % decim) { set_error("real channelizer: decimation %zu must divide the branch count %zu", decim, m); return B200C_ERR_INVALID; }
+    DevInfo di;
+    int rc = dev_info(device, di);
+    if (rc) return rc;
+    b200c_rchan *h = new (std::nothrow) b200c_rchan();
+    if (!h) { set_error("out of host memory"); return B200C_ERR_NOMEM; }
+    h->device = device; h->dtype = dtype; h->di = di;
+    DeviceGuard g(device);
+    if (!g.ok) { delete h; set_error("cudaSetDevice(%d) failed", device); return B200C_ERR_CUDA; }
+    rc = rchan_plan_create(h->plan, m, decim, di.smem_optin);
+    const double one = 1.0;   // taps {1}, as FIRFilter() (filter/FIRFilter.cpp:125)
+    if (!rc) rc = chan_set_taps(h->plan, &one, 1);
+    if (rc) { b200c_rchan_destroy(h); return rc; }
+    *out = h;
+    return B200C_OK;
+}
+
+int b200c_rchan_destroy(b200c_rchan *h)
+{
+    if (!h) return B200C_OK;
+    {
+        DeviceGuard g(h->device);
+        chan_plan_destroy(h->plan);
+    }
+    delete h;
+    return B200C_OK;
+}
+
+int b200c_rchan_set_taps(b200c_rchan *h, const double *taps, size_t ntaps)
+{
+    if (!h) return B200C_ERR_INVALID;
+    if (ntaps == 0 || !taps) { set_error("real channelizer: taps cannot be empty"); return B200C_ERR_INVALID; }
+    if (ntaps > kChanMaxTapsPerBranch * (size_t)h->plan.M) {
+        set_error("real channelizer: %zu taps exceed 16 per branch (%zu for %d branches)", ntaps, kChanMaxTapsPerBranch * (size_t)h->plan.M, h->plan.M);
+        return B200C_ERR_INVALID;
+    }
+    DeviceGuard g(h->device);
+    if (!g.ok) { set_error("cudaSetDevice(%d) failed", h->device); return B200C_ERR_CUDA; }
+    return chan_set_taps(h->plan, taps, ntaps);
+}
+
+int b200c_rchan_info(const b200c_rchan *h, size_t *m, size_t *nchan, size_t *decim, size_t *ntaps, size_t *input_require)
+{
+    if (!h) return B200C_ERR_INVALID;
+    if (m) *m = (size_t)h->plan.M;
+    if (nchan) *nchan = (size_t)h->plan.M / 2 + 1;
+    if (decim) *decim = (size_t)h->plan.D;
+    if (ntaps) *ntaps = h->plan.ntaps;
+    if (input_require) *input_require = h->plan.ntaps - 1 + (size_t)h->plan.D;
+    return B200C_OK;
+}
+
+int b200c_rchan_run(b200c_rchan *h, const void *d_in, size_t in_elems, uint64_t stream_index, void *d_out,
+                    size_t out_stride, size_t out_capacity, size_t *consumed, size_t *produced, void *stream)
+{
+    if (!h) return B200C_ERR_INVALID;
+    const size_t Km1 = h->plan.ntaps - 1, D = (size_t)h->plan.D;
+    const size_t F = in_elems >= Km1 + D ? std::min((in_elems - Km1) / D, out_capacity) : 0;
+    if (consumed) *consumed = F * D;
+    if (produced) *produced = F;
+    if (F == 0) return B200C_OK;
+    if (!d_in || !d_out) { set_error("b200c_rchan_run: null device buffer"); return B200C_ERR_INVALID; }
+    if (out_stride < F) { set_error("real channelizer: output stride %zu shorter than the %zu frames produced", out_stride, F); return B200C_ERR_INVALID; }
+    DeviceGuard g(h->device);
+    if (!g.ok) { set_error("cudaSetDevice(%d) failed", h->device); return B200C_ERR_CUDA; }
+    return rchan_launch(h->plan, h->dtype, d_in, F, stream_index, d_out, out_stride, (cudaStream_t)stream);
 }
 
 /* ------------------------------------------------------------------- synthesizer --- */

@@ -247,6 +247,60 @@ class Channelizer:
         return c.value, p.value
 
 
+class RealChannelizer:
+    """Owner of a b200c_rchan handle: one real float32 or int16 stream into M/2 + 1 baseband channels (polyphase
+    filter bank with M branches), decimated by `decim`.  Channel c is the Channelizer's channel c of the stream
+    taken as complex; the channels above M/2 are their conjugate mirrors and are not produced (include/b200comms.h
+    has the exact definition)."""
+
+    def __init__(self, dtype, m: int, decim: int, device: int = 0):
+        self.dtype = dtype_code(dtype)
+        self.m = int(m)
+        self.nchan = self.m // 2 + 1
+        self.decim = int(decim)
+        self.device = device
+        self._h = ctypes.c_void_p()
+        if self.m < 0 or self.decim < 0:
+            raise _abi.InvalidArgumentError(_abi.ERR_INVALID, "negative branch count or decimation")
+        _abi.check(_abi.lib().b200c_rchan_create(ctypes.byref(self._h), self.dtype, self.m, self.decim, device))
+
+    def close(self):
+        try:
+            if getattr(self, "_h", None) is not None and self._h:
+                _abi.lib().b200c_rchan_destroy(self._h)
+                self._h = ctypes.c_void_p()
+        except (TypeError, AttributeError):
+            pass
+
+    __del__ = close
+
+    def set_taps(self, taps):
+        t = _taps_array(taps, False)
+        _abi.check(_abi.lib().b200c_rchan_set_taps(self._h, t.ctypes.data, t.size))
+
+    def info(self):
+        """(m, nchan, decim, ntaps, input_require), nchan = m/2 + 1"""
+        m, n, d, k, req = (ctypes.c_size_t() for _ in range(5))
+        _abi.check(_abi.lib().b200c_rchan_info(self._h, ctypes.byref(m), ctypes.byref(n), ctypes.byref(d), ctypes.byref(k),
+                                               ctypes.byref(req)))
+        return m.value, n.value, d.value, k.value, req.value
+
+    def run(self, d_in, out, stream_index: int = 0, out_capacity: int | None = None, stream=None):
+        """d_in: contiguous 1-D CUDA tensor of float32 or int16 (the handle's dtype; ntaps-1 history samples first);
+        out: CUDA tensor [m/2 + 1, capacity, 2] float32, frame t of channel c lands in out[c, t].  stream_index:
+        absolute stream index of d_in[0].  Returns (consumed, produced)."""
+        assert d_in.is_cuda and d_in.is_contiguous() and d_in.dim() == 1 and d_in.dtype == torch_scalar(self.dtype)
+        assert out.is_cuda and out.is_contiguous() and out.dim() == 3 and out.shape[0] == self.nchan
+        assert out.dtype == torch_scalar(_abi.F32)
+        stride = out.shape[1]
+        cap = stride if out_capacity is None else int(out_capacity)
+        c, p = ctypes.c_size_t(), ctypes.c_size_t()
+        _abi.check(_abi.lib().b200c_rchan_run(self._h, ctypes.c_void_p(d_in.data_ptr()), d_in.numel(),
+                                              int(stream_index) & (2**64 - 1), ctypes.c_void_p(out.data_ptr()), stride, cap,
+                                              ctypes.byref(c), ctypes.byref(p), _stream_ptr(stream, d_in.device)))
+        return c.value, p.value
+
+
 class Synthesizer:
     """Owner of a b200c_synth handle: `nchan` baseband channels, interpolated by `interp`, back into one complex
     float32 stream (polyphase synthesis filter bank, the transpose of Channelizer).  Channel c is /comms/fir_filter
