@@ -21,11 +21,10 @@ import pytest
 import torch
 
 from _bank_ref import fir_count, fir_ref
+from _gpu_checks import MAX_TOL, RMS_TOL, _check, _profiled, _untouched
 
 pytestmark = pytest.mark.gpu
 
-WIN = 4096
-RMS_TOL, MAX_TOL = 1e-5, 5e-4          # float32 paths, of the channel's output RMS (north-star tolerance)
 CF64_RMS_TOL, CF64_MAX_TOL = 1e-13, 5e-12
 B200_SMS = 148
 CHUNK = 16                             # channels per reference chunk
@@ -70,17 +69,6 @@ def _path_id(nchan, n_out, ntaps):
     return kern + (f"-parts{parts}" if parts is not None else "")
 
 
-def _profiled(fn):
-    """Run fn() under torch.profiler (CUDA activities); returns (fn's result, names of the fir_* kernels that ran)."""
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        r = fn()
-        torch.cuda.synchronize()
-    names = [e.name.replace(" ", "") for e in prof.events() if str(e.device_type).endswith("CUDA")]
-    return r, [n for n in names if "fir_" in n]
-
-
 def _assert_kernels(names, pattern, what):
     assert names, f"{what}: the profiler recorded no fir kernel"
     bad = [n for n in names if not re.search(pattern, n)]
@@ -93,42 +81,6 @@ def _assert_path(names, nchan, n_out, ntaps, what):
 
 
 # ------------------------------------------------------------------------------------------------- comparison ---
-def _check(got, ref, what, chans=None, rms_tol=RMS_TOL, max_tol=MAX_TOL):
-    """got, ref: [nch, n] tensors on one device; per channel, per window of WIN outputs, relative to the channel's
-    output RMS.  A NaN anywhere fails.  chans: the channel numbers of the rows, for the report."""
-    assert got.shape == ref.shape, (what, tuple(got.shape), tuple(ref.shape))
-    nch, n = ref.shape
-    if n == 0:
-        return
-    ref = ref.to(torch.complex128 if ref.is_complex() else torch.float64)
-    d2 = (got.to(ref.dtype) - ref).abs() ** 2
-    rms = (ref.abs() ** 2).mean(dim=1).sqrt()
-    nw = -(-n // WIN)
-    d2 = torch.nn.functional.pad(d2, (0, nw * WIN - n)).view(nch, nw, WIN)
-    cnt = torch.full((nw,), float(WIN), dtype=torch.float64, device=d2.device)
-    cnt[-1] = n - (nw - 1) * WIN
-    werr = (d2.sum(-1) / cnt).sqrt() / rms[:, None]
-    wmax = d2.amax(-1).sqrt() / rms[:, None]
-    bad = ~(werr <= rms_tol) | ~(wmax <= max_tol)
-    if bool(bad.any()):
-        first = bad.nonzero()[:4].tolist()
-        rows = [f"(channel {chans[c] if chans is not None else c}, window {w}): rms {float(werr[c, w]):.2e}, "
-                f"max {float(wmax[c, w]):.2e}" for c, w in first]
-        pytest.fail(f"{what}: {int(bad.sum())} of {nch * nw} (channel, window) pairs out of tolerance "
-                    f"(rms {rms_tol}, max {max_tol}); first: " + "; ".join(rows))
-
-
-def _untouched(t, value, what):
-    """Every element of the complex tensor t still holds `value` (NaN: still NaN)."""
-    if t.numel() == 0:
-        return
-    if value != value:
-        ok = torch.isnan(torch.view_as_real(t)).all()      # both parts still NaN
-    else:
-        ok = (t == value).all()
-    assert bool(ok), f"{what}: written where nothing may be"
-
-
 def _check_bank_out(x, taps, out, produced, zero_tail, what, chans=None):
     """x: [nch, n_in] complex64 (device), taps: [nch, K] (device), out: [nch, >= produced] complex64 NaN-filled
     before the run.  Compares a chunk of channels at a time with fir_ref."""
