@@ -67,6 +67,7 @@ struct FirOsPlan {
     void *d_twf = nullptr;    // [64][64] float2: W4096^(j*t), the whole step-twiddle table
     void *d_hf1k = nullptr;   // [1024] float2: spectrum of the taps / 1024
     void *d_tw1k = nullptr;   // [32][32] float2: W1024^(j*t)
+    void *d_tw1ks = nullptr;  // [17][32] float2: W1024^(r*s(t)), fir_os32_kernel's signed step twiddles (os32_signed_twiddles)
     void *d_H = nullptr;      // general: [L*M][1024] float2 tap-phase spectra / 1024
     size_t H_floats = 0;
     // output blocks q covered by one kernel block (host-buffer chunking aligns to this)

@@ -321,7 +321,7 @@ struct FirOs32Args {
     const void *in;
     void *out;
     const void *hf;     // [nchan][1024] spectrum of the taps / 1024
-    const void *tw;     // [32][32] W1024^(j*t)
+    const void *tw;     // [17][32] signed step twiddles W1024^(r s(t)) (os32_signed_twiddles; row 0 unused)
     long long n_in, n_out;             // per channel
     long long in_stride, out_stride;   // elements between consecutive channels (filter bank)
     int nchan;
@@ -334,7 +334,12 @@ struct FirOs32Args {
 // memory -- single-channel streams only (a filter bank has one spectrum per channel)
 // EARLY (TABS form): every warp also owns a landing buffer, so the bulk copy of its NEXT block is issued as soon as the
 // current block sits in registers and has the whole block's compute time to arrive (instead of the last register pass).
+// Lanes and register indices are signed (os32_signed): lane t >= 16 takes the elements 32 m + t - 32 (mod 1024) of the
+// block, and multiplies bin t - 32 + 32 k2 (mod 1024) of the spectrum, so a step twiddle is 16 loads from the 16-row
+// table instead of 31 from the 32-row one.  Only row 0 (m = 0, k2 = 0) wraps, to the end of the block.
+// (PT is not read: the partial twiddles measured no gain here; the parameter stays in the kernel's name.)
 constexpr int kOs32Landing = 1032;   // c2 elements per landing buffer (1026 used)
+constexpr int kOs32TabElems = 1024 + 512;   // TABS: tap spectrum, then rows 1..16 of the signed twiddles
 template <int WARPS, int MINB, bool TABS = false, bool PT = kOs32PartialTwiddles, bool EARLY = false>
 __global__ void __launch_bounds__(32 * WARPS, MINB) fir_os32_kernel(const FirOs32Args a)
 {
@@ -342,12 +347,14 @@ __global__ void __launch_bounds__(32 * WARPS, MINB) fir_os32_kernel(const FirOs3
     __shared__ __align__(16) c2 Fs[TABS ? 1 : WARPS][TABS ? 1 : kOs32SmemElems];
     __shared__ __align__(8) unsigned long long bars[WARPS];
     const int t = threadIdx.x & 31, w = threadIdx.x >> 5;
+    // the lane's signed index and its element in row 0 (t, or 992 + t for the lanes that wrap)
+    const int so = os32_signed(t), s0 = so & 1023;
     c2 *F = TABS ? os32_dyn + w * kOs32SmemElems : Fs[TABS ? 0 : w];
     unsigned long long *bar = &bars[w];
     const c2 *__restrict__ tw = static_cast<const c2 *>(a.tw);
     const c2 *__restrict__ hf_tab = nullptr;
     c2 *Lb = F;                                               // where the bulk copy lands
-    if constexpr (TABS && EARLY) Lb = os32_dyn + WARPS * kOs32SmemElems + 2048 + w * kOs32Landing;
+    if constexpr (TABS && EARLY) Lb = os32_dyn + WARPS * kOs32SmemElems + kOs32TabElems + w * kOs32Landing;
     const int Km1 = a.K - 1;
     const int hop = 1024 - Km1;
     const long long nblk = (a.n_out + hop - 1) / hop;
@@ -376,26 +383,43 @@ __global__ void __launch_bounds__(32 * WARPS, MINB) fir_os32_kernel(const FirOs3
     if constexpr (TABS) {
         // Programmatic dependent launch (the host sets the attribute on this form, B200C_PDL=0 turns it off): the NEXT launch
         // in the stream may start its CTAs on the SMs this one has left, and this launch ran its own prologue -- barrier
-        // init, 16 KB of tables -- while its predecessor was still finishing; only here, before the first access to stream
+        // init, 12 KB of tables -- while its predecessor was still finishing; only here, before the first access to stream
         // data, does it wait for the predecessor to complete and flush.  Back-to-back work() calls on small buffers pay the
         // launch latency and the prologue once, not per call (DESIGN 4.10).  Both instructions are no-ops in a plain launch.
         asm volatile("griddepcontrol.launch_dependents;");
         c2 *tab = os32_dyn + WARPS * kOs32SmemElems;
         const c2 *__restrict__ hf0 = static_cast<const c2 *>(a.hf);
+        // every load of the 12 KB is issued before the first store: one memory latency, not one per element a thread
+        // copies (a launch of one block per warp waits for this prologue)
+        auto stage = [&] {
+            constexpr int kStep = 32 * WARPS, kIt = (kOs32TabElems + kStep - 1) / kStep;
+            c2 r[kIt];
+#pragma unroll
+            for (int j = 0; j < kIt; j++) {
+                const int i = (int)threadIdx.x + j * kStep;
+                if (i < kOs32TabElems) r[j] = i < 1024 ? hf0[i] : tw[i - 1024 + 32];
+            }
+#pragma unroll
+            for (int j = 0; j < kIt; j++) {
+                const int i = (int)threadIdx.x + j * kStep;
+                if (i < kOs32TabElems) tab[i] = r[j];
+            }
+        };
         if (a.pdl) {
-            for (int i = threadIdx.x; i < 1024; i += 32 * WARPS) { tab[i] = hf0[i]; tab[1024 + i] = tw[i]; }
+            stage();
             asm volatile("griddepcontrol.wait;" ::: "memory");
             if (pending && t == 0) bulk_load(Lb, src, kBulk * (unsigned)sizeof(c2), bar);
         } else {
             // plain launch: the tables are staged while the first block is in flight
             if (pending && t == 0) bulk_load(Lb, src, kBulk * (unsigned)sizeof(c2), bar);
-            for (int i = threadIdx.x; i < 1024; i += 32 * WARPS) { tab[i] = hf0[i]; tab[1024 + i] = tw[i]; }
+            stage();
         }
         __syncthreads();
-        hf_tab = tab; tw = tab + 1024;
+        hf_tab = tab; tw = tab + 1024 - 32;                   // tw[32 r + t], r = 1..16
     } else {
         if (pending && t == 0) bulk_load(Lb, src, kBulk * (unsigned)sizeof(c2), bar);
     }
+    const c2 *__restrict__ twl = tw + t;
     while (ch < a.nchan) {
         const long long base = blk * hop;
         long long nch = ch + dch, nblkpos = blk + dblk;      // this warp's next task
@@ -404,16 +428,17 @@ __global__ void __launch_bounds__(32 * WARPS, MINB) fir_os32_kernel(const FirOs3
         const c2 *__restrict__ hf = TABS ? hf_tab : static_cast<const c2 *>(a.hf) + ch * 1024;
         c2 *__restrict__ out = static_cast<c2 *>(a.out) + ch * a.out_stride;
         c2 v[32];
+        // register rev32(n1) of lane t: element 32 n1 + s(t) of the block (mod 1024)
         if (pending) {
             const int mis = (int)(((reinterpret_cast<unsigned long long>(in) >> 3) + base) & 1);
             mbar_wait(bar, parity);
             parity ^= 1;
 #pragma unroll
-            for (int n1 = 0; n1 < 32; n1++) v[rev32(n1)] = Lb[mis + 32 * n1 + t];
+            for (int n1 = 0; n1 < 32; n1++) v[rev32(n1)] = Lb[mis + (n1 ? 32 * n1 + so : s0)];
         } else {
 #pragma unroll
             for (int n1 = 0; n1 < 32; n1++) {
-                const long long g = base + 32 * n1 + t;
+                const long long g = n1 ? base + so + 32 * n1 : base + s0;
                 v[rev32(n1)] = g < a.n_in ? __ldcg(in + g) : 0ull;
             }
         }
@@ -423,26 +448,20 @@ __global__ void __launch_bounds__(32 * WARPS, MINB) fir_os32_kernel(const FirOs3
             if (pending && t == 0) bulk_load(Lb, src, kBulk * (unsigned)sizeof(c2), bar);
         }
         dft32_dit<false>(v);
-        if constexpr (PT) twiddle32<false, false>(v, tw, t);
-        else {
 #pragma unroll
-            for (int k1 = 1; k1 < 32; k1++) v[k1] = cmul_p<false>(v[k1], tw[k1 * 32 + t]);
-        }
+        for (int k1 = 1; k1 < 32; k1++) v[k1] = os32_step<false>(v[k1], twl, k1);   // * W1024^(s(k1) s(t))
         __syncwarp();
 #pragma unroll
         for (int k1 = 0; k1 < 32; k1++) F[k1 * kOs32Stride + t] = v[k1];
         __syncwarp();
 #pragma unroll
         for (int n2 = 0; n2 < 32; n2++) v[rev32(n2)] = F[t * kOs32Stride + n2];
-        dft32_dit<false>(v);
+        dft32_dit<false>(v);                                 // v[k2] = X[s(t) + 32 k2]
 #pragma unroll
-        for (int k2 = 0; k2 < 32; k2++) v[k2] = cmul_p<false>(v[k2], hf[32 * k2 + t]);
+        for (int k2 = 0; k2 < 32; k2++) v[k2] = cmul_p<false>(v[k2], hf[k2 ? 32 * k2 + so : s0]);
         dft32_dif<true>(v);
-        if constexpr (PT) twiddle32<true, true>(v, tw, t);
-        else {
 #pragma unroll
-            for (int n2 = 1; n2 < 32; n2++) v[rev32(n2)] = cmul_p<true>(v[rev32(n2)], tw[n2 * 32 + t]);
-        }
+        for (int n2 = 1; n2 < 32; n2++) v[rev32(n2)] = os32_step<true>(v[rev32(n2)], twl, n2);   // * conj W1024^(s(n2) s(t))
         __syncwarp();
 #pragma unroll
         for (int n2 = 0; n2 < 32; n2++) F[t * kOs32Stride + n2] = v[rev32(n2)];
@@ -455,18 +474,19 @@ __global__ void __launch_bounds__(32 * WARPS, MINB) fir_os32_kernel(const FirOs3
             if (pending && t == 0) bulk_load(F, src, kBulk * (unsigned)sizeof(c2), bar);
         }
         dft32_dif<true>(v);
-        c2 *o = out + (base - Km1);
+        // register rev32(n1) of lane t: circular result c[i], i = 32 n1 + s(t) (mod 1024); i >= K-1 is y[base + i - (K-1)]
+        c2 *o = out + (base - Km1), *ol = o + so;
         if (base + hop <= a.n_out) {
 #pragma unroll
             for (int n1 = 0; n1 < 32; n1++) {
-                const int i = 32 * n1 + t;
-                if (i >= Km1) __stcg(o + i, v[rev32(n1)]);
+                const int i = n1 ? 32 * n1 + so : s0;
+                if (i >= Km1) __stcg(n1 ? ol + 32 * n1 : o + s0, v[rev32(n1)]);
             }
         } else {
 #pragma unroll
             for (int n1 = 0; n1 < 32; n1++) {
-                const int i = 32 * n1 + t;
-                if (i >= Km1 && base + i - Km1 < a.n_out) __stcg(o + i, v[rev32(n1)]);
+                const int i = n1 ? 32 * n1 + so : s0;
+                if (i >= Km1 && base + i - Km1 < a.n_out) __stcg(n1 ? ol + 32 * n1 : o + s0, v[rev32(n1)]);
             }
         }
         ch = nch; blk = nblkpos;
@@ -1419,9 +1439,10 @@ int fir_os_configure(FirOsPlan &p, int dtype, const double *taps, size_t ntaps, 
             taps_spectrum(hf, 4096, taps, ntaps, complex_taps);
             if ((rc = upload(&p.d_hf, hf))) return rc;
         } else {
-            if (!p.d_tw1k) {
-                unit_root_table(tb, 1024, 32, 32, 1);
-                if ((rc = upload(&p.d_tw1k, tb))) return rc;
+            if (!p.d_tw1ks) {
+                tb.resize(2 * 32 * (size_t)kOs32SignedTwRows);
+                os32_signed_twiddles(tb.data());
+                if ((rc = upload(&p.d_tw1ks, tb))) return rc;
             }
             taps_spectrum(hf, 1024, taps, ntaps, complex_taps);
             if ((rc = upload(&p.d_hf1k, hf))) return rc;
@@ -1474,7 +1495,7 @@ int fir_os_configure(FirOsPlan &p, int dtype, const double *taps, size_t ntaps, 
 
 void fir_os_destroy(FirOsPlan &p)
 {
-    for (void **d : {&p.d_hf, &p.d_twa, &p.d_twb, &p.d_twf, &p.d_hf1k, &p.d_tw1k, &p.d_H, &p.d_hx, &p.d_tw3}) {
+    for (void **d : {&p.d_hf, &p.d_twa, &p.d_twb, &p.d_twf, &p.d_hf1k, &p.d_tw1k, &p.d_tw1ks, &p.d_H, &p.d_hx, &p.d_tw3}) {
         if (*d) cudaFree(*d);
         *d = nullptr;
     }
@@ -1652,7 +1673,7 @@ int fir_os_launch(const FirOsPlan &p, const void *d_in, size_t in_elems, void *d
     const long long nblk = (((long long)n_out + p.hop() - 1) / p.hop()) * nchan;
     if (p.N == 1024) {
         FirOs32Args a;
-        a.in = d_in; a.out = d_out; a.hf = batch ? batch->d_hf : p.d_hf1k; a.tw = p.d_tw1k;
+        a.in = d_in; a.out = d_out; a.hf = batch ? batch->d_hf : p.d_hf1k; a.tw = p.d_tw1ks;
         a.n_in = (long long)in_elems; a.n_out = (long long)n_out; a.K = p.K;
         a.nchan = nchan; a.in_stride = batch ? batch->in_stride : 0; a.out_stride = batch ? batch->out_stride : 0;
         a.spread = 0; a.pdl = 0;
@@ -1660,7 +1681,7 @@ int fir_os_launch(const FirOsPlan &p, const void *d_in, size_t in_elems, void *d
             // single stream: one persistent 12-warp CTA per SM, tap spectrum + twiddles in shared memory, a landing buffer per
             // warp (the next block is fetched a whole block ahead).  Round-1 steps, headline Gsamples/s: 12 one-warp CTAs 272,
             // persistent + shared tables 288, + landing buffers 300; partial twiddles measured no gain and are gone.
-            const size_t smem_early = sizeof(c2) * (12 * (size_t)kOs32SmemElems + 2048 + 12 * (size_t)kOs32Landing);
+            const size_t smem_early = sizeof(c2) * (12 * (size_t)kOs32SmemElems + kOs32TabElems + 12 * (size_t)kOs32Landing);
             static thread_local bool configured[16] = {false};
             int dev = 0;
             B200C_CUDA_TRY(cudaGetDevice(&dev));

@@ -16,6 +16,8 @@
 // All register indices are compile-time constants after unrolling, so the base-4 digit
 // reversal the in-place transforms need is free (it only renames registers).
 #pragma once
+#include <cmath>
+
 #include "packed.cuh"
 
 namespace b200c {
@@ -161,5 +163,34 @@ template <bool INV> B200C_HD void dft32_dif(c2 (&v)[32])
 // exchange buffer of one 1024-point transform (one warp): element (r, c) at r*33 + c
 constexpr int kOs32Stride = 33;
 constexpr int kOs32SmemElems = 32 * kOs32Stride;
+
+// Signed indices of the 32 x 32 decomposition (fir_os32_kernel).  Any index may be replaced by a representative modulo
+// 32 if its neighbour in n = 32 n1 + n2 (k = k1 + 32 k2) shifts to match, so lanes and register indices i >= 16 stand
+// for s(i) = i - 32: lane L >= 16 works on row-shifted data (element 32 m + L - 32, mod 1024), and every step twiddle
+// W1024^(s(k) s(L)) is T[|s(k)|][L] = W1024^(|s(k)| s(L)) or, for s(k) < 0, its conjugate.  |s(k)| <= 16, so one
+// 16-row table serves both directions: 16 loads per step twiddle instead of 31, the inverse taking the conjugates.
+B200C_HD constexpr int os32_signed(int i) { return i < 16 ? i : i - 32; }
+
+// v * W1024^(s(k) s(L)) (INV: its conjugate) for register index k = 1..31 of lane L; twl = T + L.  The conjugate is
+// picked by k, a compile-time constant after unrolling, so it is the operand negate of cmul_p.
+template <bool INV> B200C_HD c2 os32_step(c2 v, const c2 *twl, const int k)
+{
+    const int s = os32_signed(k);
+    return s > 0 ? cmul_p<INV>(v, twl[32 * s]) : cmul_p<!INV>(v, twl[-32 * s]);
+}
+
+// T[r][L] = W1024^(r s(L)), r = 0..16 (row 0 unused, so that the row is |s(k)|), as float2 pairs: 2 * 17 * 32 floats.
+// Computed in double and rounded once to float.
+constexpr int kOs32SignedTwRows = 17;
+inline void os32_signed_twiddles(float *tb)
+{
+    const double two_pi = 2.0 * 3.14159265358979323846264338327950288;
+    for (int r = 0; r < kOs32SignedTwRows; r++)
+        for (int L = 0; L < 32; L++) {
+            const int e = (r * os32_signed(L)) & 1023;
+            tb[2 * (r * 32 + L)] = (float)std::cos(-two_pi * e / 1024);
+            tb[2 * (r * 32 + L) + 1] = (float)std::sin(-two_pi * e / 1024);
+        }
+}
 
 } // namespace b200c
