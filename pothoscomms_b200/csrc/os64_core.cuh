@@ -111,9 +111,82 @@ template <bool INV> B200C_HD void dft64_dif(c2 (&v)[64])
 constexpr int kOs64Stride = 65;
 constexpr int kOs64SmemElems = 64 * kOs64Stride;
 
+// ------------------------------------------------------ tangent-factored butterflies ---
+// A twiddle w = W64^e (INV: its conjugate) is written as f (1 + i t) with f = Re w, t = Im w / Re w when |Re w| >= |Im w|,
+// and as f (t + i) with f = Im w, t = Re w / Im w otherwise, so that |t| <= 1.  u = b (1 + i t) or b (t + i) is then ONE
+// FFMA2 (i b is an operand swap and negate), and the scale f folds into the butterfly's add and subtract, which become
+// FFMA2 as well: a twiddled radix-2 butterfly a +- w b costs 3 instead of 4 packed instructions, a radix-4 one 11 instead
+// of 14.  The error stays that of the plain form (tools/dft32_tangent_check.cpp).  f and t are compile-time constants
+// at every call site.
+struct TanW64 {
+    float f, t;
+    bool cot;   // f (t + i) rather than f (1 + i t)
+};
+template <bool INV> B200C_HD constexpr TanW64 tan_w64(int e)
+{
+    const float c = cos64(e), s = INV ? sin64(e) : -sin64(e);
+    const bool cot = (c < 0 ? -c : c) < (s < 0 ? -s : s);
+    return cot ? TanW64{s, c / s, true} : TanW64{c, s / c, false};
+}
+// b (1 + i t) or b (t + i)
+B200C_HD c2 tan_mul(c2 b, const TanW64 w)
+{
+    float x, y;
+    upk(b, x, y);
+    return w.cot ? fma2(b, pk(w.t, w.t), pk(-y, x)) : fma2(pk(-y, x), pk(w.t, w.t), b);
+}
+
+// (a, b) <- (a + W64^e b, a - W64^e b)  (INV: conjugate twiddle)
+template <bool INV> B200C_HD void bfly2_w64(c2 &a, c2 &b, int e)
+{
+    e &= 63;
+    if (e == 0 || e == 16 || e == 48) {
+        const c2 wb = mul_w64<INV>(b, e);
+        b = sub2(a, wb);
+        a = add2(a, wb);
+        return;
+    }
+    const TanW64 w = tan_w64<INV>(e);
+    const c2 u = tan_mul(b, w);
+    b = fma2(u, pk(-w.f, -w.f), a);
+    a = fma2(u, pk(w.f, w.f), a);
+}
+
+// Decimation-in-time radix-4 butterfly with twiddles W64^e, W64^2e, W64^3e on f1, f2, f3, then the 4-point DFT.
+// e = 0 (no twiddles) or 1 <= e <= 15, so that the twiddles of f1 and f3 are not trivial: with w1 = f1 u1 / b and
+// w3 = f3 u3 / d, w1 b +- w3 d = f1 (u1 +- (f3 / f1) u3), and f1 folds into the last four adds.
+template <bool INV> B200C_HD void bfly4_w64(c2 &a, c2 &b, c2 &c, c2 &d, int e)
+{
+    if (e == 0) {
+        dft4_p<INV>(a, b, c, d);
+        return;
+    }
+    c2 p, m;   // a +- W64^2e c
+    const int e2 = (2 * e) & 63;
+    if (e2 == 16 || e2 == 48) {
+        const c2 wc = mul_w64<INV>(c, e2);
+        p = add2(a, wc);
+        m = sub2(a, wc);
+    } else {
+        const TanW64 w2 = tan_w64<INV>(e2);
+        const c2 u2 = tan_mul(c, w2);
+        p = fma2(u2, pk(w2.f, w2.f), a);
+        m = fma2(u2, pk(-w2.f, -w2.f), a);
+    }
+    const TanW64 w1 = tan_w64<INV>(e), w3 = tan_w64<INV>(3 * e);
+    const float r = w3.f / w1.f, f = w1.f;
+    const c2 u1 = tan_mul(b, w1), u3 = tan_mul(d, w3);
+    const c2 s3 = fma2(u3, pk(r, r), u1), s4 = rot_p<INV>(fma2(u3, pk(-r, -r), u1));
+    a = fma2(s3, pk(f, f), p);
+    c = fma2(s3, pk(-f, -f), p);
+    b = fma2(s4, pk(f, f), m);
+    d = fma2(s4, pk(-f, -f), m);
+}
+
 // ---------------------------------------------------------------- 32-point transforms ---
 // Radix 4, 4, 2.  Element n = q + 2 q' + 8 n'' (q < 2, q' < 4, n'' < 4) sits in register
 // rev32(n) = 16 q + 4 q' + n'' for the decimation-in-time input / decimation-in-frequency output.
+// 190 packed FMA-pipe instructions per transform (the plain form, a complex multiply per twiddle: 220).
 B200C_HD constexpr int rev32(int n) { return 16 * (n & 1) + 4 * ((n >> 1) & 3) + ((n >> 3) & 3); }
 
 template <bool INV> B200C_HD void dft32_dit(c2 (&v)[32])
@@ -125,39 +198,22 @@ template <bool INV> B200C_HD void dft32_dit(c2 (&v)[32])
 #pragma unroll
         for (int k = 0; k < 4; k++) {
             const int i = 16 * g + k;
-            v[i + 4] = mul_w64<INV>(v[i + 4], 4 * k);
-            v[i + 8] = mul_w64<INV>(v[i + 8], 8 * k);
-            v[i + 12] = mul_w64<INV>(v[i + 12], 12 * k);
-            dft4_p<INV>(v[i], v[i + 4], v[i + 8], v[i + 12]);
+            bfly4_w64<INV>(v[i], v[i + 4], v[i + 8], v[i + 12], 4 * k);   // W16^k
         }
 #pragma unroll
-    for (int k = 0; k < 16; k++) {
-        const c2 b = mul_w64<INV>(v[k + 16], 2 * k);   // W32^k
-        v[k + 16] = sub2(v[k], b);
-        v[k] = add2(v[k], b);
-    }
+    for (int k = 0; k < 16; k++) bfly2_w64<INV>(v[k], v[k + 16], 2 * k);   // W32^k
 }
 
+// The same transform with input n in v[n] and output k in v[rev32(k)]: dft32_dit on renamed registers (every index is
+// a compile-time constant, so the renaming costs no instruction).
 template <bool INV> B200C_HD void dft32_dif(c2 (&v)[32])
 {
+    c2 w[32];
 #pragma unroll
-    for (int k = 0; k < 16; k++) {
-        const c2 d = sub2(v[k], v[k + 16]);
-        v[k] = add2(v[k], v[k + 16]);
-        v[k + 16] = mul_w64<INV>(d, 2 * k);
-    }
+    for (int n = 0; n < 32; n++) w[rev32(n)] = v[n];
+    dft32_dit<INV>(w);
 #pragma unroll
-    for (int g = 0; g < 2; g++)
-#pragma unroll
-        for (int k = 0; k < 4; k++) {
-            const int i = 16 * g + k;
-            dft4_p<INV>(v[i], v[i + 4], v[i + 8], v[i + 12]);
-            v[i + 4] = mul_w64<INV>(v[i + 4], 4 * k);
-            v[i + 8] = mul_w64<INV>(v[i + 8], 8 * k);
-            v[i + 12] = mul_w64<INV>(v[i + 12], 12 * k);
-        }
-#pragma unroll
-    for (int g = 0; g < 8; g++) dft4_p<INV>(v[4 * g], v[4 * g + 1], v[4 * g + 2], v[4 * g + 3]);
+    for (int k = 0; k < 32; k++) v[rev32(k)] = w[k];
 }
 
 // exchange buffer of one 1024-point transform (one warp): element (r, c) at r*33 + c

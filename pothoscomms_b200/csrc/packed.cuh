@@ -10,6 +10,7 @@
 // The same functions compile for the host (plain float maths) so that the index logic of the
 // kernels built on them can be checked on a CPU-only box (tools/os64_host_check.cu).
 #pragma once
+#include <cmath>
 #include <cstring>
 
 #if defined(__CUDACC__)
@@ -32,10 +33,10 @@ B200C_HD c2 sub2(c2 a, c2 b) { c2 d; asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : 
 #else
 B200C_HD c2 pk(float a, float b) { float f[2] = {a, b}; c2 r; std::memcpy(&r, f, 8); return r; }
 B200C_HD void upk(c2 p, float &a, float &b) { float f[2]; std::memcpy(f, &p, 8); a = f[0]; b = f[1]; }
-B200C_HD c2 fma2(c2 a, c2 b, c2 c)
+B200C_HD c2 fma2(c2 a, c2 b, c2 c)   // one rounding, as FFMA2
 {
     float ax, ay, bx, by, cx, cy; upk(a, ax, ay); upk(b, bx, by); upk(c, cx, cy);
-    return pk(ax * bx + cx, ay * by + cy);
+    return pk(std::fma(ax, bx, cx), std::fma(ay, by, cy));
 }
 B200C_HD c2 mul2(c2 a, c2 b) { float ax, ay, bx, by; upk(a, ax, ay); upk(b, bx, by); return pk(ax * bx, ay * by); }
 B200C_HD c2 add2(c2 a, c2 b) { float ax, ay, bx, by; upk(a, ax, ay); upk(b, bx, by); return pk(ax + bx, ay + by); }
