@@ -231,6 +231,41 @@ int b200c_synth_info(const b200c_synth *h, size_t *nchan, size_t *interp, size_t
 int b200c_synth_run(b200c_synth *h, const void *d_in, size_t in_stride, size_t in_frames, uint64_t stream_index, void *d_out,
                     size_t out_capacity, size_t *consumed, size_t *produced, void *stream);
 
+/* ------------------------- real-output polyphase synthesis filter bank (one real stream out) --- */
+/* The transpose of the real-input channelizer: puts the M/2 + 1 rows c = 0 .. M/2 that b200c_rchan_run writes back
+ * into ONE real stream of float32 or int16 (what direct-IF / direct-RF DACs take).  With M = branches, N = M/2,
+ * D = interp, K = ceil(ntaps/D) and s = stream_index, the absolute stream index of d_out[0], output sample
+ * m = t D + j (j < D) is
+ *   y[t D + j] = sum_{k < K} g[j + k D] sum_{c = 0..N} w_c Re( exp(+2 pi i c (s + t D + j) / M) X_c[K-1 + t - k] ),
+ *   w_0 = w_N = 1, w_c = 2 otherwise   (g zero beyond ntaps),
+ * i.e. the real part of b200c_synth_run's output at M channels when rows M - c are conj(X_c) for 0 < c < N.  Only
+ * the real parts of rows 0 and N are read.  Only s mod M matters.  int16 output is the float32 result rounded to
+ * nearest (ties to even) and saturated to [-32768, 32767], with no other scaling: bit-identical to clamping and
+ * rounding the float32 output of the same taps and input.  Non-finite values give unspecified int16 samples.
+ * Computed as a polyphase synthesizer: the real inverse M-point DFT of each input frame packed into one M/2-point
+ * complex inverse FFT (within the frame, never two frames together), then K real-tap products per output sample.
+ *
+ * dtype (the output) B200C_F32 or B200C_I16 (else B200C_ERR_UNSUPPORTED); M a power of two in [2, 8192] (else
+ * B200C_ERR_UNSUPPORTED); D >= 1 dividing M (else B200C_ERR_INVALID).  Checked before any device call.  Taps: real
+ * doubles stored as float32, {1} after create; 1 <= ntaps <= min(16 M, 32 D), else B200C_ERR_INVALID and the old
+ * taps stay.
+ *
+ * Perfect reconstruction after b200c_rchan with D = M/2: the complex pair's recipe (b200c_synth above) unchanged. */
+typedef struct b200c_rsynth b200c_rsynth;
+int b200c_rsynth_create(b200c_rsynth **out, int dtype, size_t m, size_t interp, int device);
+int b200c_rsynth_destroy(b200c_rsynth *h);
+int b200c_rsynth_set_taps(b200c_rsynth *h, const double *taps, size_t ntaps);
+/* nchan = M/2 + 1 input rows; input_require = K frames per row */
+int b200c_rsynth_info(const b200c_rsynth *h, size_t *m, size_t *nchan, size_t *interp, size_t *ntaps, size_t *input_require);
+/* d_in: M/2 + 1 rows of complex float32 in the real channelizer's output layout, frame i of row c at
+ * d_in[c * in_stride + i] for i < in_frames; the first K-1 frames of every row are history.
+ * F = min(in_frames - (K-1), out_capacity / D), 0 when in_frames < K; *consumed = F frames per row, *produced = F D
+ * samples of the handle's dtype, written to d_out[0 .. F D) and nowhere else; d_out may start at any element offset.
+ * Null buffers (with F > 0) or in_stride < in_frames -> B200C_ERR_INVALID.  Stateless, asynchronous on `stream`,
+ * one kernel launch; an output sample's value does not depend on how the stream was cut into calls (bit for bit). */
+int b200c_rsynth_run(b200c_rsynth *h, const void *d_in, size_t in_stride, size_t in_frames, uint64_t stream_index,
+                     void *d_out, size_t out_capacity, size_t *consumed, size_t *produced, void *stream);
+
 /* ------------------------------------------------------------------------- /comms/fft --- */
 typedef struct b200c_fft b200c_fft;
 

@@ -68,6 +68,12 @@ SYMBOLS = {
     "b200c_synth_info": (_i, [_vp, _psz, _psz, _psz, _psz]),
     # stream_index is a uint64, as for b200c_chan_run
     "b200c_synth_run": (_i, [_vp, _vp, _sz, _sz, ctypes.c_uint64, _vp, _sz, _psz, _psz, _vp]),
+    "b200c_rsynth_create": (_i, [_pvp, _i, _sz, _sz, _i]),
+    "b200c_rsynth_destroy": (_i, [_vp]),
+    "b200c_rsynth_set_taps": (_i, [_vp, _vp, _sz]),
+    "b200c_rsynth_info": (_i, [_vp, _psz, _psz, _psz, _psz, _psz]),
+    # stream_index is a uint64, as for b200c_synth_run
+    "b200c_rsynth_run": (_i, [_vp, _vp, _sz, _sz, ctypes.c_uint64, _vp, _sz, _psz, _psz, _vp]),
     "b200c_fft_create": (_i, [_pvp, _i, _sz, _i, _i]),
     "b200c_fft_destroy": (_i, [_vp]),
     "b200c_fft_info": (_i, [_vp, _psz, _pi]),

@@ -356,6 +356,64 @@ class Synthesizer:
         return c.value, p.value
 
 
+class RealSynthesizer:
+    """Owner of a b200c_rsynth handle: the M/2 + 1 baseband channels of a RealChannelizer (polyphase filter bank with
+    M branches), interpolated by `interp`, back into one real float32 or int16 stream.  The output is the real part of
+    the Synthesizer's at M channels with rows M - c taken as conj(row c); int16 output is rounded to nearest and
+    saturated (include/b200comms.h has the exact definition)."""
+
+    def __init__(self, dtype, m: int, interp: int, device: int = 0):
+        self.dtype = dtype_code(dtype)
+        self.m = int(m)
+        self.nchan = self.m // 2 + 1
+        self.interp = int(interp)
+        self.device = device
+        self._h = ctypes.c_void_p()
+        if self.m < 0 or self.interp < 0:
+            raise _abi.InvalidArgumentError(_abi.ERR_INVALID, "negative branch count or interpolation")
+        _abi.check(_abi.lib().b200c_rsynth_create(ctypes.byref(self._h), self.dtype, self.m, self.interp, device))
+
+    def close(self):
+        try:
+            if getattr(self, "_h", None) is not None and self._h:
+                _abi.lib().b200c_rsynth_destroy(self._h)
+                self._h = ctypes.c_void_p()
+        except (TypeError, AttributeError):
+            pass
+
+    __del__ = close
+
+    def set_taps(self, taps):
+        t = _taps_array(taps, False)
+        _abi.check(_abi.lib().b200c_rsynth_set_taps(self._h, t.ctypes.data, t.size))
+
+    def info(self):
+        """(m, nchan, interp, ntaps, input_require), nchan = m/2 + 1, input_require = ceil(ntaps / interp) frames"""
+        m, n, d, k, req = (ctypes.c_size_t() for _ in range(5))
+        _abi.check(_abi.lib().b200c_rsynth_info(self._h, ctypes.byref(m), ctypes.byref(n), ctypes.byref(d), ctypes.byref(k),
+                                                ctypes.byref(req)))
+        return m.value, n.value, d.value, k.value, req.value
+
+    def run(self, d_in, out, stream_index: int = 0, in_frames: int | None = None, out_capacity: int | None = None,
+            stream=None):
+        """d_in: CUDA tensor [m/2 + 1, stride, 2] float32, frame i of row c in d_in[c, i] (the RealChannelizer's output
+        layout; the first ceil(ntaps/interp)-1 frames are history); out: contiguous 1-D CUDA tensor of float32 or int16
+        (the handle's dtype), which may start at any element.  stream_index: absolute stream index of out[0].
+        Returns (consumed frames per row, produced samples)."""
+        import torch
+        assert d_in.is_cuda and d_in.is_contiguous() and d_in.dtype == torch.float32
+        assert d_in.dim() == 3 and d_in.shape[0] == self.nchan and d_in.shape[2] == 2
+        assert out.is_cuda and out.is_contiguous() and out.dim() == 1 and out.dtype == torch_scalar(self.dtype)
+        stride = d_in.shape[1]
+        frames = stride if in_frames is None else int(in_frames)
+        cap = out.numel() if out_capacity is None else int(out_capacity)
+        c, p = ctypes.c_size_t(), ctypes.c_size_t()
+        _abi.check(_abi.lib().b200c_rsynth_run(self._h, ctypes.c_void_p(d_in.data_ptr()), stride, frames,
+                                               int(stream_index) & (2**64 - 1), ctypes.c_void_p(out.data_ptr()), cap,
+                                               ctypes.byref(c), ctypes.byref(p), _stream_ptr(stream, d_in.device)))
+        return c.value, p.value
+
+
 class Fft:
     """Owner of a b200c_fft handle (the FFTAux of one /comms/fft block)."""
 
