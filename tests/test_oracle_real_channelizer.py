@@ -9,10 +9,15 @@ import pytest
 from _chan_oracle import channelize
 
 
-def real_channelize(x, h, M, D, s=0, frames=None):
-    """Rows 0 .. M/2 of the complex channelizer's definition on the real samples x.  x is made complex first: a real
-    array handed to channelize() would be read as interleaved (re, im) pairs."""
-    return channelize(np.asarray(x, dtype=np.float64).astype(np.complex128), h, M, D, s, frames)[: M // 2 + 1]
+def real_channelize(x, h, M, D, s=0, frames=None, channels=None):
+    """Rows 0 .. M/2 (or the listed ``channels``, each <= M/2) of the complex channelizer's definition on the real
+    samples x.  x is made complex first: a real array handed to channelize() would be read as interleaved (re, im)
+    pairs."""
+    xc = np.asarray(x, dtype=np.float64).astype(np.complex128)
+    if channels is None:
+        return channelize(xc, h, M, D, s, frames)[: M // 2 + 1]
+    assert all(0 <= c <= M // 2 for c in channels)
+    return channelize(xc, h, M, D, s, frames, channels)
 
 
 CASES = [
